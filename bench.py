@@ -255,6 +255,27 @@ def run_reference(args):
     return 0
 
 
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, s, blocks, block_ids, nblocks_total, with_norms, np):
+    """What the timed step hands its caller: the residual dw of every owned cell of each block (float64, layout
+    (i, j, k, variable)) and the two residual norms.  A block whose dw exceeds its share of the 64 MiB budget is
+    written as a fixed sample: flat indices drawn with seed 0, sorted; the same sample for every build."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BUDGET_BYTES // nblocks_total - 4096
+    for q, (hb, b) in enumerate(zip(blocks, block_ids)):
+        dw = np.ascontiguousarray(s.downloadResidual(q)[hb.d.owned()], dtype=np.float64)
+        if dw.nbytes > share:
+            pick = np.sort(np.random.default_rng(0).choice(dw.size, share // 8, replace=False))
+            np.save(os.path.join(out_dir, "residual_block%d_sample.npy" % b), dw.reshape(-1)[pick])
+        else:
+            np.save(os.path.join(out_dir, "residual_block%d.npy" % b), dw)
+    norms = np.asarray(s.getResNorms(), dtype=np.float64)   # every rank: the norms are reduced over the job
+    if with_norms:
+        np.save(os.path.join(out_dir, "residual_norms.npy"), norms)
+
+
 def workload_name(shape, nblocks):
     return "C2 %dx%dx%d RANS-SA residual (blocketteRes), %d block(s)" % (tuple(shape) + (nblocks,))
 
@@ -464,7 +485,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--shape", type=int, nargs=3, default=list(C2))
     ap.add_argument("--no-scaling-sections", action="store_true", help="skip the C3 strong-scaling and C5 matvec sections")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -551,6 +575,9 @@ def main():
     ms_total = timed_steps(step, args.steps)
     launches = s.launchCount() - n0
     barrier()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, s, blocks, grid.local_blocks(rank), grid.nblocks, rank == 0, np)
+        barrier()
     # ---- e2e through the vector API with pinned host buffers -------------------
     nvec = s.getStateSize()
     h_state = torch.empty(nvec, dtype=torch.float64).pin_memory()

@@ -58,16 +58,21 @@ def test_c2_residual_matches_oracle_and_reference(cuda_lib):
     host_tot = np.sum(r ** 2)
     assert abs(norms[0] - host_rho) <= 1e-12 * host_rho
     assert abs(norms[1] - host_tot) <= 1e-12 * host_tot
-    # the reference's own routines, when the translated build travelled with the snapshot
+    # the reference's own routines (where the translated library is absent: the oracle's residual, once it matches the
+    # recorded digest of the reference's bit for bit)
+    import refgold as gold
     from oracle import refblockette as rb
-    if rb.available():
+
+    def reference():
         hr = hb.copy()
         orr = Oracle(hr, prm)
         orr.pressure(False); orr.lam_viscosity(False); orr.eddy_viscosity(False)
         orr.apply_turb_bc(True); orr.apply_flow_bc(True)
-        rdw = rb.residual_core(hr, prm).a["dw"]
-        for l in range(6):
-            assert rel_l2(dw[ow + (l,)], rdw[ow + (l,)]) < 1e-10, l
+        return rb.residual_core(hr, prm)
+
+    rdw = gold.value("dw", gold.run(reference), lambda r: r.a["dw"][ow], ho.dw[ow])
+    for l in range(6):
+        assert rel_l2(dw[ow + (l,)], rdw[..., l]) < 1e-10, l
 
 
 def test_c2_free_stream_preservation(cuda_lib):
